@@ -2,14 +2,15 @@
 """bench.py — the headline measurement: 4K yuv420p -> rgb24 swscale frames/s (BASELINE.json configs[1]),
 with the batched 8x8 IDCT (configs[2]) reported beside it, on N GPUs of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 One step = one pass of the hot path over one batch of 256 synthetic 4K frames per GPU (weak scaling: every rank
 converts its own batch, no data-path collective; the optional NCCL gather at the mux boundary is reported separately).
 Rank 0 prints ONE JSON line.  `value` is device-resident throughput (CUDA events on the launching stream, max over
 ranks); `e2e` is the same metric through the C-ABI host entry point with pinned HOST buffers, H2D and D2H copies inside
 the timed region.  --impl reference times the reference's own CPU implementation (oracle/_ref/libffref.so when it was
-built from /root/reference, else the oracle port) with all host threads on a bounded sample of the same workload.
+built, else the oracle port) with all host threads on a bounded sample of the same workload.
+--dump-outputs DIR writes what the headline's last timed step computed (rank 0's rgb24 frames) as DIR/*.npy, see dump_outputs().
 """
 import argparse
 import json
@@ -744,6 +745,23 @@ def extra_paths(args, dev, stream, g, world, barrier, reduce_max, peak, devidx):
 
 
 
+DUMP_SAMPLES = 1 << 22                         # bytes of the batch's rgb24 output sampled into the dump (16 MB as float32)
+
+
+def dump_outputs(out_dir, OUT):
+    """The headline's output batch [BATCH, H, W*3] uint8, too large to store whole (6.4 GB): frame 0 and frame BATCH-1 at 1/4 scale
+    in both directions (every 4th row and pixel) and DUMP_SAMPLES bytes at fixed, seeded positions of the whole batch, as float32."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    px = OUT.view(BATCH, H4K, W4K, 3)
+    for i in (0, BATCH - 1):
+        np.save(os.path.join(out_dir, f"sws_rgb24_frame{i}_sub4.npy"), px[i, ::4, ::4].float().cpu().numpy())
+    idx = torch.randint(0, OUT.numel(), (DUMP_SAMPLES,), generator=torch.Generator().manual_seed(1234)).sort().values
+    np.save(os.path.join(out_dir, "sws_rgb24_batch_sample.npy"), OUT.view(-1)[idx.to(OUT.device)].float().cpu().numpy())
+    np.save(os.path.join(out_dir, "sws_rgb24_batch_sample_index.npy"), idx.double().numpy())
+
+
 def run_b200(args, rank, world, local_rank, placement=None):
     import torch
     import torch.distributed as dist
@@ -809,6 +827,8 @@ def run_b200(args, rank, world, local_rank, placement=None):
     sampler = ClockSampler(local_rank)
     sampler.start()
     total_ms, kern_ms, launches = timed_sws(FLAGS_FATE, args.steps, args.warmup, True)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, OUT)
     fps = world * BATCH * args.steps / (total_ms / 1e3)
     ach = FRAME_BYTES * BATCH / (kern_ms / 1e3) / 1e9
     roof = {"bound": "hbm", "achieved": ach, "peak": peak, "unit": "GB/s", "frac": ach / peak, "peak_source": peak_src,
@@ -1119,7 +1139,10 @@ def main():
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the headline's last timed step's output (sampled) as DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

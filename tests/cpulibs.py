@@ -84,6 +84,57 @@ def have_ref():
     return os.path.exists(REF_SO)
 
 
+REF_RECORD_DIR = os.path.join(ROOT, "tests", "golden", "ref")
+
+
+def _digest(a):
+    """dtype, shape and contents of an array in 8 hex digits: enough to tell a changed output from the recorded one"""
+    import hashlib
+    a = np.ascontiguousarray(np.asarray(a))
+    return hashlib.sha256(f"{a.dtype.str} {a.shape}".encode() + a.tobytes()).hexdigest()[:8]
+
+
+class RefRecord:
+    """What the compiled reference produced at each comparison point of one test, in the order the test compares, stored as
+    digests in tests/golden/ref/<test>.txt.  With oracle/_ref built, same(got, fn) calls fn and compares live, and the reference's
+    value must also match the stored digest (FFREF_RECORD=1 rewrites the file instead).  Without it, got is compared with the
+    stored digest, so a checkout without the reference keeps every comparison (got must then have the reference value's dtype)."""
+
+    def __init__(self, name):
+        self.path = os.path.join(REF_RECORD_DIR, name + ".txt")
+        self.live = have_ref()
+        self.recording = self.live and os.environ.get("FFREF_RECORD") == "1"
+        self.stored = None if self.recording or not os.path.exists(self.path) else open(self.path).read().split("\n")[:-1]
+        self.seen = []
+
+    def usable(self):
+        return self.live or self.stored is not None
+
+    def same(self, got, fn):
+        """True when `got` equals what fn() (a call of the reference) returns; fn is called only when the reference is built"""
+        i = len(self.seen)
+        if self.live:
+            r = np.asarray(fn())
+            self.seen.append(_digest(r))
+            assert self.stored is None or (i < len(self.stored) and self.stored[i] == self.seen[i]), \
+                ("the reference no longer matches " + self.path, i)
+            if not np.array_equal(np.asarray(got), r):
+                return False
+            assert _digest(got) == self.seen[i], ("equal values of another dtype or shape: stored digests could not be checked", i)
+            return True
+        assert i < len(self.stored), ("more comparisons than " + self.path + " holds", i)
+        self.seen.append(self.stored[i])
+        return _digest(got) == self.stored[i]
+
+    def close(self):
+        if self.recording:
+            os.makedirs(REF_RECORD_DIR, exist_ok=True)
+            with open(self.path, "w") as f:
+                f.write("".join(s + "\n" for s in self.seen))
+        elif self.stored is not None:
+            assert len(self.seen) == len(self.stored), ("fewer comparisons than " + self.path + " holds", len(self.seen), len(self.stored))
+
+
 def ref():
     global _ref
     if _ref is None:

@@ -456,7 +456,8 @@ def test_sws_nv_destinations(device):
             out = gpu_sws_planar(device, 640, 360, dw, dh, FATE, y, uv, uv, src_fmt=cl.PIX_FMT_NV12, dst_fmt=df)
             exp = cl.orc_sws_planar(640, 360, dw, dh, FATE, y, uv, uv, src_fmt=cl.PIX_FMT_NV12, dst_fmt=df)
             assert all(np.array_equal(p, q) for p, q in zip(out, exp)), ("nv12 source", dw, df)
-    fg.check_all(functools.partial(gpu_sws, device), functools.partial(gpu_sws_planar, device), rgb_sources=True, nv_dest=True)     # all 59 FATE sums
+    if cl.have_nut() and os.path.exists(cl.VIDEOGEN):                # FATE's frames and NUT muxer come from the reference build
+        fg.check_all(functools.partial(gpu_sws, device), functools.partial(gpu_sws_planar, device), rgb_sources=True, nv_dest=True)     # all 59 FATE sums
     # the encoder feed: bgra 1080p -> nv12 (packed RGB source kernels too), and the batched device entry point with two destination planes
     src = cl.rgb_frame(1920, 1080, 2900, 4)
     out = gpu_sws_planar(device, 1920, 1080, 1920, 1080, FATE, src, src, src, src_fmt=cl.PIX_FMT_BGRA, dst_fmt=cl.PIX_FMT_NV12)
