@@ -174,6 +174,9 @@ void orc_h264_weight(int idx, uint8_t *block, ptrdiff_t stride, int height, int 
 void orc_h264_biweight(int idx, uint8_t *dst, const uint8_t *src, ptrdiff_t stride, int height, int log2_denom,
                        int weightd, int weights, int offset);
 int  orc_h264chroma(int avg, int idx, uint8_t *dst, const uint8_t *src, ptrdiff_t stride, int h, int x, int y);
+/* b200_h264chroma_batch_device's operation list (op byte: bit0 avg, bits1-2 width index; xy byte: x | y << 3); -1 at an invalid op */
+int  orc_h264chroma_batch(int64_t n, const uint8_t *op, const uint8_t *h, const uint8_t *xy, uint8_t *dstbase, const int64_t *dst_off,
+                          const uint8_t *srcbase, const int64_t *src_off, ptrdiff_t stride);
 
 /* ------------------------------------------------------------------ tx (float FFT / MDCT, power-of-two) */
 typedef struct OrcTx OrcTx;

@@ -270,6 +270,17 @@ int orc_h264chroma(int avg, int idx, uint8_t *dst, const uint8_t *src, ptrdiff_t
     return 0;
 }
 
+/* a list of operations, as b200_h264chroma_batch_device takes it (op byte: bit0 avg, bits1-2 width index; xy byte: x | y << 3),
+ * applied in list order; -1 at the first invalid operation (the ones before it are done), else 0 */
+int orc_h264chroma_batch(int64_t n, const uint8_t *op, const uint8_t *h, const uint8_t *xy, uint8_t *dstbase, const int64_t *dst_off,
+                         const uint8_t *srcbase, const int64_t *src_off, ptrdiff_t stride)
+{
+    for (int64_t i = 0; i < n; i++)
+        if (orc_h264chroma(op[i] & 1, (op[i] >> 1) & 3, dstbase + dst_off[i], srcbase + src_off[i], stride, h[i], xy[i] & 7, (xy[i] >> 3) & 7) < 0)
+            return -1;
+    return 0;
+}
+
 void orc_emulated_edge_mc(uint8_t *buf, const uint8_t *src, ptrdiff_t buf_linesize, ptrdiff_t src_linesize,
                           int block_w, int block_h, int src_x, int src_y, int w, int h)
 {

@@ -71,6 +71,8 @@ def oracle():
             L.orc_h264_biweight.restype = None
         if hasattr(L, "orc_h264chroma"):
             L.orc_h264chroma.argtypes = [C.c_int, C.c_int, u8p, u8p, C.c_ssize_t, C.c_int, C.c_int, C.c_int]
+        if hasattr(L, "orc_h264chroma_batch"):
+            L.orc_h264chroma_batch.argtypes = [C.c_int64, u8p, u8p, u8p, u8p, i64p, u8p, i64p, C.c_ssize_t]
         if hasattr(L, "orc_tx_open"):
             L.orc_tx_open.restype = C.c_void_p
             L.orc_tx_open.argtypes = [C.c_int, C.c_int, C.c_int, C.c_float, C.c_uint]

@@ -606,7 +606,8 @@ def test_tx_rdft_batch_vs_oracle(device, n):
 
 def test_tx_linearity_1m_batch(device):
     """BASELINE config 5 size (a large batch of len-1024 transforms): FFT(a) + FFT(b) ~= FFT(a + b) and Parseval,
-    size-independent properties at a size the oracle cannot cover; plus unsupported configurations are refused loudly."""
+    size-independent properties of a 200 000-transform batch; plus unsupported configurations are refused loudly.  The bit-exact
+    comparison with the oracle over several rounds of the persistent grid, for every tx_r16 size, is test_batch_rounds_gpu.py's."""
     import torch
     import ffmpeg_b200 as fb
     from ffmpeg_b200 import tx

@@ -72,6 +72,35 @@ def test_h264chroma_oracle_vs_ref(refrec):
         assert refrec.same(d2, ref_out), (avg, idx, x, y, h)
 
 
+def test_h264chroma_batch_oracle_equals_single_calls():
+    """orc_h264chroma_batch (the device entry's operation list) applies each operation as orc_h264chroma does, in list order:
+    overlapping destinations, avg on top of earlier results, every phase / width / height, unaligned offsets"""
+    O = cl.oracle()
+    rng = np.random.default_rng(31)
+    W, H, n = 80, 72, 3000
+    src = rng.integers(0, 256, (H, W), dtype=np.uint8)
+    dst0 = rng.integers(0, 256, (H, W), dtype=np.uint8)
+    idx = rng.integers(0, 3, n)
+    op = ((idx << 1) | rng.integers(0, 2, n)).astype(np.uint8)
+    h = np.array([rng.choice(((2, 4, 8, 16), (2, 4, 8), (2, 4))[i]) for i in idx], np.uint8)
+    xy = (np.arange(n) % 64).astype(np.uint8)
+    doff = (rng.integers(0, H - 16, n) * W + rng.integers(0, W - 8, n)).astype(np.int64)
+    soff = (rng.integers(0, H - 17, n) * W + rng.integers(0, W - 9, n)).astype(np.int64)
+    exp = dst0.copy()
+    for i in range(n):
+        assert O.orc_h264chroma(int(op[i]) & 1, int(op[i]) >> 1, C.cast(exp.ctypes.data + int(doff[i]), cl.u8p),
+                                C.cast(src.ctypes.data + int(soff[i]), cl.u8p), W, int(h[i]), int(xy[i]) & 7, int(xy[i]) >> 3) == 0
+    got = dst0.copy()
+    assert O.orc_h264chroma_batch(n, cl.ptr(op), cl.ptr(h), cl.ptr(xy), cl.ptr(got), cl.ptr(doff, cl.i64p), cl.ptr(src),
+                                  cl.ptr(soff, cl.i64p), W) == 0
+    assert np.array_equal(got, exp), int((got != exp).sum())
+    assert not np.array_equal(got, dst0)
+    bad = op.copy()
+    bad[5] = 3 << 1                                                # table entry [3] does not exist
+    assert O.orc_h264chroma_batch(n, cl.ptr(bad), cl.ptr(h), cl.ptr(xy), cl.ptr(dst0.copy()), cl.ptr(doff, cl.i64p), cl.ptr(src),
+                                  cl.ptr(soff, cl.i64p), W) == -1
+
+
 def test_emulated_edge_mc_oracle_golden():
     from cases import EDGE_PIC, EDGE_CASES
     g = np.load(os.path.join(G, "edge.npz"))
